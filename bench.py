@@ -748,6 +748,22 @@ class near_gpu:
         return False
 
 
+DUMP_ROWS = 3_000_000  # float64 values + their row indices: 48 MB per dump, small enough to keep two runs side by side
+
+
+def dump_outputs(out_dir, name, v):
+    """Writes the device vector v, the result a caller of the timed path receives, to out_dir/<name>.npy as float64.  A longer
+    vector than DUMP_ROWS is sampled, the same rows on every run (seed 0); their indices go to out_dir/<name>_rows.npy."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    if v.numel() > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_ROWS, replace=False))
+        v = v[torch.from_numpy(rows).to(v.device)]
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy().astype(np.float64))
+
+
 def verify_transport(op, x, n_total, world, rank, dev):
     """One step and two chained steps of a row-block operator: every rank's copy of the gathered vector must be bit-identical to
     every other rank's (probes of each block are exchanged over NCCL), and the first result must not change under the steps
@@ -801,6 +817,9 @@ def main():
     ap.add_argument("--ctas", type=int, default=-1)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step to DIR/<name>.npy (y; x_next for N>1), float64, at most "
+                         f"{DUMP_ROWS} seeded sample rows with their indices in DIR/<name>_rows.npy")
     ap.add_argument("--no-secondary", action="store_true", help="N=1: skip the configs[2] / configs[3] workloads")
     ap.add_argument("--collective", default="auto",
                     choices=["auto", "pipelined", "pipelined_mc", "pipelined_sm", "fused", "multicast", "multicast_fwd", "nccl"],
@@ -811,6 +830,8 @@ def main():
     ap.add_argument("--chunks", type=int, default=8)
     ap.add_argument("--push-ctas", type=int, default=32)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     # libraries (NCCL prints its version line) must not pollute stdout: the JSON line is the only thing on it
@@ -1004,6 +1025,11 @@ def main():
     if world > 1:
         dist.barrier()
     launches = lib.b200sp_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        if op is None:
+            dump_outputs(args.dump_outputs, "y", y)
+        else:  # every rank holds the whole gathered vector
+            dump_outputs(args.dump_outputs, "x_next", op.x_next)
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)

@@ -9,6 +9,7 @@ import pytest
 
 from crs_cases import MERGE_CASES, random_matrix, spadd_dense_check
 from helpers import kk_matrix
+from ref_digests import Case
 
 
 @pytest.mark.parametrize("case", sorted(MERGE_CASES))
@@ -84,24 +85,28 @@ def test_spadd_sorted_equals_unsorted_on_strict_input(oracle):
 @pytest.mark.parametrize("n,kmax", [(0, 10), (1, 10), (2, 3), (17, 4), (1000, 16), (5000, 70000), (3000, 2**31 - 1)])
 def test_row_sort_equals_reference_radix_sort(oracle, n, kmax):
     """The restated per-row sort of sort_crs_matrix (host path) equals the reference's own SerialRadixSort2 -- compiled from
-    common/src/KokkosKernels_Sorting.hpp in place (oracle/_ref) -- bit for bit, ties included (stability)."""
-    if oracle.ref is None or not hasattr(oracle.ref, "kkref_radix_sort2_u32_f64"):
-        pytest.skip("oracle/_ref not built")
+    common/src/KokkosKernels_Sorting.hpp in place (oracle/_ref) -- bit for bit, ties included (stability); without oracle/_ref,
+    against its recorded output."""
+    live = oracle.ref is not None and hasattr(oracle.ref, "kkref_radix_sort2_u32_f64")
+    gold = Case(live, "radix_sort2", n, kmax)
     rng = np.random.default_rng(n + kmax % 97)
     ci = rng.integers(0, kmax, n).astype(np.int32)
     v = rng.uniform(-1, 1, n)
     rp = np.array([0, n], dtype=np.int32)
     eci, ev = ci.copy(), v.copy()
     oracle.sort_crs_stable(rp, eci, ev)
-    keys, perm = ci.astype(np.uint32), v.copy()
-    oracle.ref_radix_sort2(keys, perm)
-    assert np.array_equal(eci.astype(np.uint32), keys) and np.array_equal(ev, perm)
     ids = np.arange(n, dtype=np.int32)  # graph sort with a payload that exposes the order of ties
     eci2, eid = ci.copy(), ids.copy()
     oracle.sort_crs_stable(rp, eci2, eid)
-    keys2, perm2 = ci.astype(np.uint32), ids.copy()
-    oracle.ref_radix_sort2(keys2, perm2)
-    assert np.array_equal(eid, perm2)
+    gold.add(eci.astype(np.uint32), ev, eid)
+    if live:
+        keys, perm = ci.astype(np.uint32), v.copy()
+        oracle.ref_radix_sort2(keys, perm)
+        assert np.array_equal(eci.astype(np.uint32), keys) and np.array_equal(ev, perm)
+        keys2, perm2 = ci.astype(np.uint32), ids.copy()
+        oracle.ref_radix_sort2(keys2, perm2)
+        assert np.array_equal(eid, perm2)
+    gold.check()
 
 
 @pytest.mark.parametrize("sorted_input", [True, False])
@@ -109,14 +114,18 @@ def test_row_sort_equals_reference_radix_sort(oracle, n, kmax):
 def test_spadd_numeric_equals_reference_functors(oracle, sorted_input, m, n, lo, hi):
     """The restated numeric phase of spadd equals the reference's own functors -- sparse/impl/KokkosSparse_spadd_numeric_impl.hpp
     compiled from the reference tree in place (oracle/_ref) -- bit for bit, for sorted / merged and for unsorted input
-    (rows longer than the column count repeat columns)."""
-    if oracle.ref is None or not hasattr(oracle.ref, "kkref_spadd_sorted_numeric_f64"):
-        pytest.skip("oracle/_ref not built")
+    (rows longer than the column count repeat columns); without oracle/_ref, against its recorded output."""
+    live = oracle.ref is not None and hasattr(oracle.ref, "kkref_spadd_sorted_numeric_f64")
+    gold = Case(live, "spadd_numeric", sorted_input, m, n, lo, hi)
     from crs_cases import random_matrix
 
     hi_eff = min(hi, n) if sorted_input else hi  # sorted + merged input has distinct columns
     A = random_matrix(m, n, min(lo, hi_eff), hi_eff, sorted_input, seed=1)
     B = random_matrix(m, n, min(lo, hi_eff), hi_eff, sorted_input, seed=2)
     got = oracle.spadd(*A, 0.3, *B, -1.7, sorted_input)
-    ref = oracle.ref_spadd_numeric(*A, 0.3, *B, -1.7, sorted_input)
-    assert np.array_equal(got[0], ref[0]) and np.array_equal(got[1], ref[1]) and np.array_equal(got[2], ref[2])
+    assert not np.isnan(got[2]).any()
+    gold.add(*got)
+    if live:
+        ref = oracle.ref_spadd_numeric(*A, 0.3, *B, -1.7, sorted_input)
+        assert np.array_equal(got[0], ref[0]) and np.array_equal(got[1], ref[1]) and np.array_equal(got[2], ref[2])
+    gold.check()
